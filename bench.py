@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the GRU/BiLSTM hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]                  # this repo's CUDA path
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]  # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]  # reference CPU path (oracle port)
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      # one rank per GPU, NCCL
 
@@ -531,27 +531,28 @@ def run_ours(args) -> None:
     torch.cuda.synchronize()
 
     # ---- capture one CUDA graph per resident input batch ---------------------------------------------
-    graphs, use_graph = [], not args.no_graph
+    graphs, graph_outs, use_graph = [], [], not args.no_graph
     if use_graph:
         try:
             pool = None
             for i in range(N_ROTATE):
                 g = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g, pool=pool):
-                    train_step(*dev_in[i])
+                    graph_outs.append(train_step(*dev_in[i]))
                 pool = g.pool()
                 graphs.append(g)
         except Exception as exc:  # e.g. NCCL capture unsupported: fall back to eager launches
             if rank == 0:
                 print(f"[bench] CUDA-graph capture failed ({type(exc).__name__}: {exc}); running eager", file=sys.stderr)
-            use_graph, graphs = False, []
+            use_graph, graphs, graph_outs = False, [], []
             torch.cuda.synchronize()
 
     def run_step(i: int):
+        """One train step; returns the model output tensor the step wrote (a graph's static output when replayed)."""
         if use_graph:
             graphs[i % N_ROTATE].replay()
-        else:
-            train_step(*dev_in[i % N_ROTATE])
+            return graph_outs[i % N_ROTATE]
+        return train_step(*dev_in[i % N_ROTATE])
 
     _log(f"graphs captured: {use_graph}; launches/step {launches_per_step}")
     # ---- (A) device-resident throughput: W warm-up + exactly K timed steps ----------------------------
@@ -566,11 +567,13 @@ def run_ours(args) -> None:
     _barrier()
     e0.record()
     for i in range(K):
-        run_step(W + i)
+        out = run_step(W + i)
     e1.record()
     _barrier()
     ms_total = _max_over_ranks(e0.elapsed_time(e1), dev)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # before the e2e leg below trains the model further
+        _dump_outputs(args.dump_outputs, {"out": out, "loss": loss_buf})
     ms_per_step = ms_total / K
     value = B_PER_GPU * n_gpus * K / (ms_total * 1e-3)
 
@@ -810,6 +813,17 @@ def run_ours(args) -> None:
     _teardown(graphs, e2e_graphs, world, fused)
 
 
+def _dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write what the last timed step returned to its caller as ``out_dir/<name>.npy`` in float32, so that two builds
+    run with the same arguments (hence the same seeded inputs and weights) can be compared output for output."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+    _log(f"outputs of the last timed step written to {out_dir}: {sorted(arrays)}")
+
+
 def _teardown(graphs, e2e_graphs, world: int, fused=None) -> None:
     """Normal interpreter exit (the driver's exit hook records which .so files this process loaded).
 
@@ -903,7 +917,14 @@ def main() -> None:
                     help="data-parallel gradient exchange of the fused step: in-kernel NVLink peer stores (peer: wait at "
                          "the end of the step; peer_async: send now, sum + Adam at the start of the next step beside "
                          "the encoders, flushed after the last step) or NCCL")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0: model output [B,2] and "
+                         "loss) as DIR/out.npy and DIR/loss.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     _protect_stdout()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":

@@ -3,7 +3,8 @@
 The reference scripts cannot be imported (they np.load absent Features/*.npz at import time and import librosa /
 allennlp / tensorflow, audio_gru_whole.py:19-20, fuse_net_whole.py:10-16), but their model classes are
 self-contained: this module parses a script, extracts the wanted ``ClassDef`` nodes and executes just those
-with torch in scope. Works only where /root/reference exists (this build container, not the GPU box).
+with torch in scope. Works only where a checkout of the reference is at ``B200RNN_REFERENCE_ROOT``; the tests never
+need it (they compare against what oracle/make_golden.py recorded from it under tests/golden/).
 """
 from __future__ import annotations
 
@@ -16,7 +17,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 from torch.autograd import Variable
 
-REFERENCE_ROOT = os.environ.get("B200RNN_REFERENCE_ROOT", "/root/reference/DepressionCollected")
+REFERENCE_ROOT = os.environ.get("B200RNN_REFERENCE_ROOT", "")
 
 FILES = {
     "audio_clf": "Classification/audio_gru_whole.py",
@@ -29,7 +30,7 @@ FILES = {
 
 
 def available() -> bool:
-    return os.path.isdir(REFERENCE_ROOT)
+    return bool(REFERENCE_ROOT) and os.path.isdir(REFERENCE_ROOT)
 
 
 def load_classes(key: str, names: Iterable[str], extra_globals: Dict | None = None) -> Dict[str, type]:

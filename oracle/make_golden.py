@@ -1,6 +1,6 @@
-"""ORACLE tooling — generates tests/golden/*.npz from the REFERENCE's own classes (run in the build container).
+"""ORACLE tooling — generates tests/golden/*.npz from the REFERENCE's own classes.
 
-    python oracle/make_golden.py            # needs /root/reference; writes tests/golden/
+    B200RNN_REFERENCE_ROOT=<reference>/DepressionCollected python oracle/make_golden.py   # writes tests/golden/
 
 Each fixture is produced by executing the reference ``ClassDef``s (oracle/ast_loader.py) on CPU with torch
 {torch_version}; weights and inputs are regenerated from names (oracle/params.py), so a fixture holds only small
@@ -133,9 +133,53 @@ def fuse(case: str, key: str, regression: bool, B: int, T: int) -> None:
                              torch=torch.__version__))
 
 
+def live_forward(case: str, key: str, cls_name: str, cfg: dict, shape, head: str) -> None:
+    """The reference class's eval() forward and its parameter names, for checking the restated class against it.
+    Also records the forward with the head's final activation removed: a regression head's ReLU maps every row of
+    some of these cases to 0, which alone would pin nothing."""
+    cls = ast_loader.load_classes(key, [cls_name])[cls_name]
+    torch.manual_seed(0)
+    model = cls(cfg)
+    params.fill_module(model)
+    model.eval()
+    x = params.inputs_for(case, shape)
+    with torch.no_grad():
+        out = model(x)
+        getattr(model, head)[-1] = nn.Identity()
+        pre = model(x)
+    _save(case, {"out": out.numpy(), "pre_activation": pre.numpy()},
+          dict(case=case, ref=ast_loader.FILES[key], cls=cls_name, cfg=cfg, shape=list(shape), head=head,
+               names=[n for n, _ in model.named_parameters()], torch=torch.__version__))
+
+
+def dropin_build(case: str) -> None:
+    """What the reference's classes construct once ``b200rnn.install()`` has rebound nn.GRU / nn.LSTM: the recurrent
+    module's class, every parameter's name and shape, and which parameters the reference's own init leaves at 0."""
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
+                                    "icassp2022-depression_b200"))
+    import b200rnn
+
+    built = {}
+    try:
+        b200rnn.install()
+        for key, cls_name, cfg, attr in (("audio_clf", "AudioBiLSTM", AUDIO_CLF, "lstm_net_audio"),
+                                         ("text_clf", "TextBiLSTM", TEXT_CLF, "lstm_net")):
+            torch.manual_seed(0)
+            model = ast_loader.load_classes(key, [cls_name])[cls_name](cfg)
+            rnn = getattr(model, attr)
+            built[key] = dict(
+                ref=ast_loader.FILES[key], cls=cls_name, attr=attr,
+                rnn_class=f"{type(rnn).__module__}.{type(rnn).__qualname__}",
+                params=[[n, list(p.shape)] for n, p in model.named_parameters()],
+                zero=[n for n, p in model.named_parameters() if float(p.detach().abs().max()) == 0.0])
+    finally:
+        b200rnn.uninstall()
+    _save(case, {}, dict(case=case, built=built, torch=torch.__version__))
+
+
 def main() -> None:
     if not ast_loader.available():
-        raise SystemExit("reference tree not found; fixtures can only be generated in the build container")
+        raise SystemExit("reference tree not found; set B200RNN_REFERENCE_ROOT to its DepressionCollected directory")
     torch.set_num_threads(1)
     single_modal("audio_clf_b3_t5", "audio_clf", "AudioBiLSTM", AUDIO_CLF, (3, 5, 256), "ce")
     single_modal("text_clf_b3_t6", "text_clf", "TextBiLSTM", TEXT_CLF, (3, 6, 1024), "ce")
@@ -147,6 +191,11 @@ def main() -> None:
     rnn_boundary("lstm_boundary_b5_t17", "text_clf", "TextBiLSTM", TEXT_CLF, "lstm_net", (5, 17, 1024), True)
     fuse("fuse_clf_b3_t3", "fuse_clf", False, 3, 3)
     fuse("fuse_reg_b3_t3", "fuse_reg", True, 3, 3)
+    live_forward("live_audio_clf_b4_t6", "audio_clf", "AudioBiLSTM", AUDIO_CLF, (4, 6, 256), "fc_audio")
+    live_forward("live_text_clf_b4_t6", "text_clf", "TextBiLSTM", TEXT_CLF, (4, 6, 1024), "fc_out")
+    live_forward("live_audio_reg_b4_t3", "audio_reg", "AudioBiLSTM", AUDIO_REG, (4, 3, 256), "fc_audio")
+    live_forward("live_text_reg_b4_t3", "text_reg", "TextBiLSTM", TEXT_REG, (4, 3, 1024), "fc_out")
+    dropin_build("dropin_build")
 
 
 if __name__ == "__main__":

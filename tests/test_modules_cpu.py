@@ -100,22 +100,29 @@ def test_unsupported_features_raise():
 
 
 def test_reference_classes_build_on_the_dropin_when_installed():
-    """The reference's own ClassDefs (AST-loaded, not copied) construct B200 modules after install()."""
-    from oracle import ast_loader, make_golden as mg
+    """After install(), model code that calls nn.GRU / nn.LSTM builds B200 modules. The restated reference classes
+    (oracle/ref_models.py) are built that way and must come out as the reference's own ClassDefs did when they were
+    built the same way (tests/golden/dropin_build.npz: recurrent module class, parameter names and shapes, and the
+    parameters its init leaves at 0)."""
+    from conftest import load_golden
+    from oracle import make_golden as mg, ref_models
 
-    if not ast_loader.available():
-        pytest.skip("/root/reference only exists in the build container")
+    _, meta = load_golden("dropin_build")
     try:
         b200rnn.install()
-        cls = ast_loader.load_classes("audio_clf", ["AudioBiLSTM"])["AudioBiLSTM"]
-        model = cls(mg.AUDIO_CLF)
+        model = ref_models.RefAudio(mg.AUDIO_CLF)
         assert isinstance(model.lstm_net_audio, b200rnn.GRU)
-        cls_t = ast_loader.load_classes("text_clf", ["TextBiLSTM"])["TextBiLSTM"]
-        model_t = cls_t(mg.TEXT_CLF)  # runs xavier init over the B200 LSTM's parameters (text_bilstm_whole.py:37-43)
+        model_t = ref_models.RefText(mg.TEXT_CLF)  # xavier init over the B200 LSTM (text_bilstm_whole.py:37-43)
         assert isinstance(model_t.lstm_net, b200rnn.LSTM)
-        assert float(model_t.lstm_net.bias_ih_l0.abs().max()) == 0.0
+        assert float(model_t.lstm_net.bias_ih_l0.detach().abs().max()) == 0.0
     finally:
         b200rnn.uninstall()
+    for key, m in (("audio_clf", model), ("text_clf", model_t)):
+        want = meta["built"][key]
+        rnn = getattr(m, want["attr"])
+        assert f"{type(rnn).__module__}.{type(rnn).__qualname__}" == want["rnn_class"], key
+        assert [[n, list(p.shape)] for n, p in m.named_parameters()] == want["params"], key
+        assert [n for n, p in m.named_parameters() if float(p.detach().abs().max()) == 0.0] == want["zero"], key
 
 
 def test_fused_shell_entry_points_reject_host_tensors():

@@ -1,12 +1,11 @@
-"""CPU tests pinning the ORACLE: numpy restatement vs the executed dependency (torch.nn.GRU / nn.LSTM), restated
-model shells vs the golden fixtures recorded from the reference's own classes, and — where /root/reference
-exists — vs those classes executed live."""
+"""CPU tests pinning the ORACLE: numpy restatement vs the executed dependency (torch.nn.GRU / nn.LSTM) and restated
+model shells vs the golden fixtures recorded from the reference's own classes."""
 import numpy as np
 import pytest
 import torch
 
 from conftest import load_golden
-from oracle import ast_loader, params, ref_models
+from oracle import params, ref_models
 from oracle.rnn_numpy import NumpyRNN
 
 FUSE_CFG = dict(text_embed_size=1024, text_hidden_dims=128, rnn_layers=2, dropout=0.3, num_classes=2,
@@ -170,7 +169,6 @@ def test_numpy_oracle_reproduces_reference_rnn_boundary(case, kind):
         _close(arrays["grad:" + n], torch.from_numpy(g), 1e-5, n)
 
 
-@pytest.mark.skipif(not ast_loader.available(), reason="/root/reference only exists in the build container")
 @pytest.mark.parametrize("key,name,cls,regression,shape", [
     ("audio_clf", "AudioBiLSTM", ref_models.RefAudio, False, (4, 6, 256)),
     ("text_clf", "TextBiLSTM", ref_models.RefText, False, (4, 6, 1024)),
@@ -178,13 +176,18 @@ def test_numpy_oracle_reproduces_reference_rnn_boundary(case, kind):
     ("text_reg", "TextBiLSTM", ref_models.RefText, True, (4, 3, 1024)),
 ])
 def test_ref_models_match_reference_live(key, name, cls, regression, shape):
-    from oracle import make_golden as mg
-
-    cfg = {"audio_clf": mg.AUDIO_CLF, "text_clf": mg.TEXT_CLF, "audio_reg": mg.AUDIO_REG, "text_reg": mg.TEXT_REG}[key]
-    theirs = ast_loader.load_classes(key, [name])[name](cfg)
-    mine = cls(cfg, regression=regression)
-    assert [n for n, _ in theirs.named_parameters()] == [n for n, _ in mine.named_parameters()]
-    mine.load_state_dict(theirs.state_dict())
-    theirs.eval(), mine.eval()
-    x = torch.randn(*shape)
-    assert torch.allclose(theirs(x), mine(x), atol=1e-6)
+    """The restated classes against the reference's own classes executed on the same weights and inputs (their
+    parameter names and eval() outputs, with and without the head's final activation, recorded by
+    oracle/make_golden.py)."""
+    case = f"live_{key}_b{shape[0]}_t{shape[1]}"
+    arrays, meta = load_golden(case)
+    assert meta["cls"] == name and meta["shape"] == list(shape)
+    mine = cls(meta["cfg"], regression=regression)
+    assert [n for n, _ in mine.named_parameters()] == meta["names"]
+    params.fill_module(mine)
+    mine.eval()
+    x = params.inputs_for(case, meta["shape"])
+    with torch.no_grad():
+        assert np.abs(mine(x).numpy() - arrays["out"]).max() <= 1e-6
+        getattr(mine, meta["head"])[-1] = torch.nn.Identity()
+        assert np.abs(mine(x).numpy() - arrays["pre_activation"]).max() <= 1e-6
