@@ -10,7 +10,7 @@ import os
 from ctypes import POINTER, c_char_p, c_float, c_int, c_int32, c_int64, c_size_t, c_uint32, c_uint64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# B200RNN_LIB: load another build of the SAME library (e.g. the -DB200RNN_TRACE build used by tools/trace_rec*.py)
+# B200RNN_LIB: load another build of the SAME library (e.g. the -DB200RNN_TRACE build used by tools/trace_rec.py)
 LIB_PATH = os.environ.get("B200RNN_LIB") or os.path.join(os.path.dirname(_HERE), "lib", "libb200rnn.so")
 
 GRU, LSTM = 0, 1

@@ -124,11 +124,9 @@ struct ScratchLayout {
   // backward
   size_t b_dgates[2], b_dghn[2], b_wt[2], b_bpart[2], b_dy, b_gemm;
   size_t b_gemm_bytes;
-  // tcgen05 backward GEMMs: dense TF32 hi/lo splits of the operands (hi at the offset, lo right behind it); the names
-  // keep their round-1 "T" although nothing is transposed any more (MN-major operands, gemm_tc.cu)
-  size_t b_tc_dg, b_tc_dgT, b_tc_hnT, b_tc_xT, b_tc_yT, b_tc_wT, b_tc_part;
+  // tcgen05 backward GEMMs: dense TF32 hi/lo splits of the operands (hi at the offset, lo right behind it)
+  size_t b_tc_dg, b_tc_hn, b_tc_x, b_tc_y, b_tc_w, b_tc_part;
   size_t b_tc_part_bytes;
-  long long b_ldk;  // leading dimension of the transposed operands: T*B rounded up to a multiple of 4
   size_t b_dxln, b_lnpart;  // fused LayerNorm backward: dense d/dLN(x) [TB][I], per-CTA column partials
   size_t b_total;
 };
@@ -177,14 +175,11 @@ void make_scratch(const Dims& d, ScratchLayout* s) {
   off += align_up(gb / sizeof(float) + 1, ALIGN_F);
   {
     const size_t Imax = d.I > (int)d.DH ? (size_t)d.I : d.DH;
-    const size_t ldk = (d.TB + 3) / 4 * 4;
-    s->b_ldk = (long long)ldk;
-    s->b_tc_dg = off;   off += align_up(2 * d.TB * d.GH, ALIGN_F);
-    s->b_tc_dgT = off;  off += align_up(2 * d.GH * ldk, ALIGN_F);
-    s->b_tc_hnT = off;  off += align_up(2 * (size_t)d.H * ldk, ALIGN_F);
-    s->b_tc_xT = off;   off += align_up(2 * Imax * ldk, ALIGN_F);
-    s->b_tc_yT = off;   off += align_up(2 * (size_t)d.H * ldk, ALIGN_F);
-    s->b_tc_wT = off;   off += align_up(2 * Imax * d.GH, ALIGN_F);
+    s->b_tc_dg = off;  off += align_up(2 * d.TB * d.GH, ALIGN_F);
+    s->b_tc_hn = off;  off += align_up(2 * d.TB * d.H, ALIGN_F);
+    s->b_tc_x = off;   off += align_up(2 * d.TB * Imax, ALIGN_F);
+    s->b_tc_y = off;   off += align_up(2 * d.TB * d.H, ALIGN_F);
+    s->b_tc_w = off;   off += align_up(2 * d.GH * Imax, ALIGN_F);
     s->b_tc_part = off;
     s->b_tc_part_bytes = (size_t)160 * 128 * 128 * sizeof(float);  // <= (#SMs / tiles) * M * N
     off += align_up(s->b_tc_part_bytes / sizeof(float), ALIGN_F);
@@ -566,17 +561,15 @@ B200RNN_API int b200rnn_backward_fused(const b200rnn_desc* desc, const float* x,
     const bool ln_l0 = (l == 0) && fused_ln;
     const bool want_dx = (l > 0) || (dx != nullptr) || (ln_l0 && (dln_gamma || dln_beta));
     // ---- tcgen05 3xTF32 path for the wgrad / dgrad GEMMs (falls back to the FFMA kernel per GEMM) -------------
-    const long long ldk = sl.b_ldk;
     const bool tc_l = tc_available() && (Il % 128 == 0);
     // Operands whose contraction index (t,b) is their ROW index - X_l, dG, h_prev, dn*r - go to the tensor cores as
     // MN-major tiles (gemm_tc.cu): they only need the dense TF32 hi/lo split, no transposing pass (round 1 transposed
     // every one of them: 10 passes, 8 % of the c2 train step).
-    float* xS = S + sl.b_tc_xT;  // [TB][Il] hi, then lo
+    float* xS = S + sl.b_tc_x;  // [TB][Il] hi, then lo
     if (tc_l) {  // X_l, shared by both directions
       rc = tc_split(in, in_rows, (int)d.TB, Il, xS, xS + d.TB * (size_t)Il, st);
       if (rc) return rc;
     }
-    (void)ldk;
     for (int k = 0; k < d.D; ++k) {
       const float* const* pp = params + (size_t)(l * d.D + k) * 4;
       float* const* gp = dparams + (size_t)(l * d.D + k) * 4;
@@ -590,7 +583,7 @@ B200RNN_API int b200rnn_backward_fused(const b200rnn_desc* desc, const float* x,
       bool done_dwih = (dw_ih == nullptr), done_dwhh = (dw_hh == nullptr), done_dx = !want_dx;
       if (tc_l) {
         float* dGs = S + sl.b_tc_dg;   // [TB][GH] hi, then lo: MN-major A of the wgrads AND K-major A of the dgrad
-        float* hnS = S + sl.b_tc_hnT;  // [TB][H]   (GRU: dn * r)
+        float* hnS = S + sl.b_tc_hn;   // [TB][H]   (GRU: dn * r)
         const TcOperand opX{xS, xS + d.TB * (size_t)Il, (long long)Il, true};
         // the tcgen05 epilogue stores float4: a gradient target that is not 16-byte aligned (a view into a caller's
         // flat bucket behind an odd-sized tensor) takes the FFMA GEMM below instead of failing
@@ -622,7 +615,7 @@ B200RNN_API int b200rnn_backward_fused(const b200rnn_desc* desc, const float* x,
         if (tc_whh) {
           // dW_hh = sum_t dGh[t]^T h_{prev(t)}: rows are (t,b) flattened time-major, so the one-step shift is a ROW
           // offset of B (forward: dG[t] with y[t-1]; reverse: dG[t] with y[t+1]); rows beyond Kp read as zero (TMA)
-          float* yS = S + sl.b_tc_yT;  // [TB][H]
+          float* yS = S + sl.b_tc_y;  // [TB][H]
           rc = tc_split(bp.y + (long long)k * d.H, tb_rows(bp.y_st, bp.y_sb, d.B), (int)d.TB, d.H, yS,
                         yS + d.TB * (size_t)d.H, st);
           if (rc) return rc;
@@ -650,7 +643,7 @@ B200RNN_API int b200rnn_backward_fused(const b200rnn_desc* desc, const float* x,
           done_dwhh = true;
         }
         if (tc_dx) {  // dX_l (+)= dG[TB, GH] * W_ih[GH, Il]: A K-major (the same split of dG), B = W_ih as it lies (MN-major)
-          float* wS = S + sl.b_tc_wT;   // [GH][Il] hi, then lo
+          float* wS = S + sl.b_tc_w;   // [GH][Il] hi, then lo
           rc = tc_split(pp[0], simple_rows(Il), (int)d.GH, Il, wS, wS + d.GH * (size_t)Il, st);
           if (rc) return rc;
           const TcOperand opA{dGs, dGs + d.TB * d.GH, (long long)d.GH, false};

@@ -17,9 +17,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void fence_mbar_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
-__device__ __forceinline__ void fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
                : "memory");
@@ -88,14 +85,6 @@ __device__ __forceinline__ uint32_t mapa(uint32_t local_smem_addr, uint32_t rank
   uint32_t r;
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_smem_addr), "r"(rank));
   return r;
-}
-__device__ __forceinline__ void st_cluster_f32(uint32_t cluster_addr, float v) {
-  asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(cluster_addr), "f"(v) : "memory");
-}
-__device__ __forceinline__ void st_cluster_v4(uint32_t cluster_addr, float4 v) {
-  asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(cluster_addr), "f"(v.x), "f"(v.y),
-               "f"(v.z), "f"(v.w)
-               : "memory");
 }
 
 // st.async: 16-byte store into a peer CTA's shared memory that also completes 16 bytes of the transaction

@@ -46,8 +46,6 @@ struct RecBwdParams {
 int rec_bwd_max_slices(int B);
 
 int launch_rec_fwd(const RecFwdParams& p, cudaStream_t stream);
-// tensor-core forward recurrence (rnn_rec_tc.cu); false = shape not covered, caller uses the FFMA kernel
-bool launch_rec_fwd_tc(const RecFwdParams& p, cudaStream_t stream, int* rc);
 int launch_rec_bwd(RecBwdParams& p, cudaStream_t stream);
 
 }  // namespace b200rnn

@@ -724,18 +724,11 @@ bool try_bwd(RecBwdParams& p, cudaStream_t s, bool force, int* rc) {
   return true;
 }
 
-int env_variant(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return v ? atoi(v) : dflt;
-}
-
 // Batch-size-aware dispatch (measured on one box, GRU H=256, T=120, per layer launch; profiles/README.md):
-//   B = 128 : FFMA <C=4,BS=4> 222 us (215 us with the batch-paired FFMA2 form) | tcgen05 recurrence 354 us
+//   B = 128 : FFMA <C=4,BS=4> 222 us (215 us with the batch-paired FFMA2 form)
 //   B =  64 : FFMA <C=4,BS=4> 215 us (64 CTAs: 43 % of the chip) | FFMA <C=4,BS=2> 175 us (128 CTAs, half the FFMA per step)
-//   B <= 48 : FFMA <C=4,BS=4> 209 us | tcgen05 ~205-215 us | FFMA <C=4,BS=2> 170 us
-// so: clusters of 2 batch rows whenever they fit one wave (B <= ~72), clusters of 4 above, and the tensor-core
-// recurrence only when forced (B200RNN_REC_TC=1) - it is bound by the 8-CTA all-to-all of the state, not by math.
-bool rec_tc_preferred(const RecFwdParams&) { return false; }
+//   B <= 48 : FFMA <C=4,BS=4> 209 us | FFMA <C=4,BS=2> 170 us
+// so: clusters of 2 batch rows whenever they fit one wave (B <= ~72), clusters of 4 above.
 }  // namespace
 
 // smallest BS any backward config uses is 2
@@ -747,17 +740,12 @@ int rec_bwd_max_slices(int B) { return (B + 1) / 2; }
 int launch_rec_fwd(const RecFwdParams& p, cudaStream_t s) {
   int rc = B200RNN_OK;
   if (p.B <= 0 || p.T <= 0) return rc;
-  // The tcgen05 recurrence (rnn_rec_tc.cu) is parity-green but never the fastest choice any more (rec_tc_preferred());
-  // B200RNN_REC_TC=1 forces it (A/B runs, tests/test_gpu_tc_rec.py).
-  static const int rec_tc = env_variant("B200RNN_REC_TC", -1);
-  if ((rec_tc == 1 || (rec_tc < 0 && rec_tc_preferred(p))) && launch_rec_fwd_tc(p, s, &rc)) return rc;
   // One tuned config per shape (B200, round-1/2 A/B runs in profiles/README.md) plus a wider-batch fallback that runs
   // in several waves when the batch needs more clusters than fit the chip.
   if (p.mode == B200RNN_GRU && p.H == 256) {
     // half-filled chip (B <= 74, e.g. BASELINE c2 with B = 64): clusters of 2 batch rows use twice the SMs with half the
     // FFMA work per step (all three gate blocks in shared memory, 4 warps per CTA)
-    static const int bs2 = env_variant("B200RNN_GRU_BS2", 1);  // =0: A/B switch
-    if (bs2 && p.B <= 74 && try_fwd<B200RNN_GRU, 256, 4, 2, 16, 8, 0>(p, s, false, &rc)) return rc;
+    if (p.B <= 74 && try_fwd<B200RNN_GRU, 256, 4, 2, 16, 8, 0>(p, s, false, &rc)) return rc;
     // batch-paired FFMA2 (rnn_core.cuh dots_chunk2b): 215 us at B=128, T=120 against 222 us for the k-paired form on
     // the same box. The same change measured SLOWER for the 2-row clusters (0.408 vs 0.397 ms per 2-layer forward at
     // B=64) and with two gate blocks in registers (0.549 vs 0.539 ms), so only this config uses it.
@@ -793,8 +781,7 @@ int launch_rec_bwd(RecBwdParams& p, cudaStream_t s) {
   // K across all 32 lanes with 8 units per lane halves the redundant reads of the [BS][G*H] gradient vector, which
   // (not the weights) dominates the shared-memory traffic of the backward contraction: 303 -> 278 us (GRU H=256)
   if (p.mode == B200RNN_GRU && p.H == 256) {
-    static const int bs2 = env_variant("B200RNN_GRU_BS2", 1);
-    if (bs2 && p.B <= 74 && try_bwd<B200RNN_GRU, 256, 4, 2, 16, 8, 0>(p, s, false, &rc)) return rc;
+    if (p.B <= 74 && try_bwd<B200RNN_GRU, 256, 4, 2, 16, 8, 0>(p, s, false, &rc)) return rc;
     if (try_bwd<B200RNN_GRU, 256, 4, 4, 32, 8, 1>(p, s, false, &rc)) return rc;
     try_bwd<B200RNN_GRU, 256, 8, 8, 32, 4, 1>(p, s, true, &rc);
     return rc;

@@ -34,6 +34,8 @@ def test_workspace_bytes_scale_with_the_problem():
     T, B, H = 120, 128, 256
     expect = 4 * T * B * (2 * 4 * H + 2 * H)
     assert expect <= big[0] <= expect * 1.01 + 4096
+    # scratch: 18 [T,B,H] blocks (dG, dn*r, dy, dLN(x), hi/lo of dG, dn*r, X, h) + ~1.2 of GEMM partials and weights
+    assert big[1] <= 20 * 4 * T * B * H
     lstm = _lib.workspace_bytes(_lib.Desc(_lib.LSTM, 64, 30, 1024, 256, 2, 2, 1, 0.0, 0))
     assert lstm[0] >= 4 * 30 * 64 * (2 * 2 * 5 * 256 + 2 * 256)
 

@@ -1,6 +1,6 @@
 """Static checks on the SASS of the built library (cuobjdump, no GPU).
 
-* the Blackwell instructions the design claims are really there (tcgen05 MMA / TMEM load+store / commit, TMA tensor
+* the Blackwell instructions the design claims are really there (tcgen05 MMA / TMEM load / commit, TMA tensor
   and bulk copies, st.async, packed FFMA2);
 * two code-generation pitfalls found with the profiler in round 1 stay fixed:
     - a tcgen05.mma / TMA issue whose operands the compiler cannot prove warp-uniform is wrapped in an
@@ -45,15 +45,15 @@ def _has(ops, prefix):
 
 def test_expected_blackwell_instructions_are_present(functions):
     all_ops = [o for ops in functions.values() for o in ops]
-    for prefix, what in [("UTCHMMA", "tcgen05.mma"), ("LDTM", "tcgen05.ld"), ("STTM", "tcgen05.st"),
-                         ("UTCBAR", "tcgen05.commit"), ("UTMALDG", "TMA tensor load"), ("UBLKCP", "TMA bulk copy"),
-                         ("STAS", "st.async"), ("FFMA2", "packed fp32 FMA"), ("SYNCS", "mbarrier")]:
+    for prefix, what in [("UTCHMMA", "tcgen05.mma"), ("LDTM", "tcgen05.ld"), ("UTCBAR", "tcgen05.commit"),
+                         ("UTMALDG", "TMA tensor load"), ("UBLKCP", "TMA bulk copy"), ("STAS", "st.async"),
+                         ("FFMA2", "packed fp32 FMA"), ("SYNCS", "mbarrier")]:
         assert _has(all_ops, prefix), f"no {prefix} ({what}) in the library"
 
 
 def test_tensor_core_issue_stays_on_the_uniform_datapath(functions):
     tc = {n: ops for n, ops in functions.items() if _has(ops, "UTCHMMA") or _has(ops, "UTMALDG")}
-    assert len(tc) >= 4, sorted(tc)   # GEMM + three tensor-core recurrence instantiations
+    assert len(tc) >= 1, sorted(tc)   # the 3xTF32 GEMM
     for name, ops in tc.items():
         assert not _has(ops, "BRA.U.ANY"), f"{name}: tcgen05 / TMA issue inside a register-broadcast loop"
 

@@ -1,7 +1,6 @@
-"""CPU emulation of the operand splits the tcgen05 kernels use, to pin the precision claims made in
-csrc/gemm_tc.cu (3xTF32: hi*hi + lo*hi + hi*lo) and csrc/rnn_rec_tc.cu (A_hi x tf32(h) + A_hi x (h - tf32(h)) +
-bf16(A_lo) x bf16(h)) independently of any GPU: with exact accumulation the split products must reproduce the fp32
-product far inside the 1e-5 parity budget, and a plain single-TF32 product must NOT (which is why the split exists).
+"""CPU emulation of the operand split the tcgen05 GEMM uses, to pin the precision claim made in csrc/gemm_tc.cu
+(3xTF32: hi*hi + lo*hi + hi*lo) independently of any GPU: with exact accumulation the split product must reproduce the
+fp32 product far inside the 1e-5 parity budget, and a plain single-TF32 product must NOT (which is why the split exists).
 The tensor core's truncating fp32 accumulate is a separate, measured effect (gemm_tc.cu header)."""
 import numpy as np
 
@@ -10,13 +9,6 @@ def tf32_rna(x):
     """cvt.rna.tf32.f32: keep 10 mantissa bits, round to nearest, ties away from zero (sign-magnitude add)."""
     u = np.asarray(x, dtype=np.float32).view(np.uint32)
     return ((u + np.uint32(0x1000)) & np.uint32(0xFFFFE000)).view(np.float32)
-
-
-def bf16_rn(x):
-    """cvt.rn.bf16.f32 (round to nearest even), returned as float32."""
-    u = np.asarray(x, dtype=np.float32).view(np.uint32)
-    bias = ((u >> np.uint32(16)) & np.uint32(1)) + np.uint32(0x7FFF)
-    return ((u + bias) & np.uint32(0xFFFF0000)).view(np.float32)
 
 
 def _case(seed, M, N, K, wscale):
@@ -30,10 +22,8 @@ def test_rounding_helpers_are_what_the_ptx_conversions_do():
     x = np.float32(1.0) + np.float32(2.0 ** -11)                    # exactly half an ulp of tf32 above 1.0
     assert tf32_rna(x) == np.float32(1.0 + 2.0 ** -10)              # ties away from zero
     assert tf32_rna(-x) == np.float32(-(1.0 + 2.0 ** -10))
-    assert bf16_rn(np.float32(1.0 + 2.0 ** -8)) == np.float32(1.0)  # tie -> even
-    assert bf16_rn(np.float32(1.0 + 3 * 2.0 ** -8)) == np.float32(1.0 + 2.0 ** -6)
     v = np.float32(0.123456789)
-    assert abs(tf32_rna(v) - v) <= abs(v) * 2.0 ** -11 and abs(bf16_rn(v) - v) <= abs(v) * 2.0 ** -8
+    assert abs(tf32_rna(v) - v) <= abs(v) * 2.0 ** -11
 
 
 def test_3xtf32_split_reproduces_the_fp32_product_and_single_tf32_does_not():
@@ -48,19 +38,3 @@ def test_3xtf32_split_reproduces_the_fp32_product_and_single_tf32_does_not():
     assert np.abs(split - exact).max() / scale < 5e-7               # dropped lo*lo ~ 2^-22
     assert np.abs(single - exact).max() / scale > 2e-5              # plain TF32 misses the 1e-5 budget
 
-
-def test_recurrence_split_with_bf16_remainder_stays_inside_the_budget():
-    a, h, exact = _case(1, 96, 9, 256, 0.0625)
-    ah = tf32_rna(a)
-    al_bf = bf16_rn(a - ah)                                          # A_lo kept as bf16 on chip
-    hh = tf32_rna(h)
-    hl = h - hh
-    h_bf = bf16_rn(h)
-    d64 = lambda x, y: x.astype(np.float64) @ y.astype(np.float64).T  # noqa: E731
-    got = d64(ah, hh) + d64(ah, hl) + d64(al_bf, h_bf)
-    err = np.abs(got - exact).max()
-    # per term the bf16 rounding of the 2^-11-sized remainders is 2^-19 relative; over K = 256 random-sign terms of
-    # size ~0.06 x 0.6 that is ~7e-7 absolute on a pre-activation: ~10x fp32 summation noise, 14x inside the budget
-    assert err < 2e-6, err
-    # the same product with the remainder terms dropped is two orders worse
-    assert np.abs(d64(ah, hh) - exact).max() > 50 * err

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Small shapes through every recurrence variant, for compute-sanitizer (memcheck / racecheck):
     compute-sanitizer --tool memcheck python tools/sanitize_paths.py
-    B200RNN_REC_TC=1 compute-sanitizer --tool racecheck python tools/sanitize_paths.py
-    B200RNN_GRU_BS2=0 compute-sanitizer --tool memcheck python tools/sanitize_paths.py rnn   # recurrence only, 4-row GRU clusters
+    compute-sanitizer --tool memcheck python tools/sanitize_paths.py rnn   # recurrence only
+The GRU H=256 case runs at B = 9 (2-row clusters) and B = 80 (4-row clusters, above the 74-row cut).
 """
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -11,21 +11,22 @@ import torch, b200rnn
 from torch.nn.utils.rnn import pack_padded_sequence
 dev = torch.device("cuda:0")
 torch.manual_seed(0)
-for kind, I, H, L, bi in (("gru", 64, 256, 2, False), ("lstm", 64, 128, 2, True), ("gru", 32, 128, 1, True), ("lstm", 32, 256, 1, False)):
+for kind, I, H, L, bi, B in (("gru", 64, 256, 2, False, 9), ("lstm", 64, 128, 2, True, 9), ("gru", 32, 128, 1, True, 9),
+                             ("lstm", 32, 256, 1, False, 9), ("gru", 64, 256, 2, False, 80)):
     cls = b200rnn.GRU if kind == "gru" else b200rnn.LSTM
     m = cls(I, H, num_layers=L, bidirectional=bi, batch_first=True, dropout=0.3 if L > 1 else 0.0).to(dev).train()
-    B, T = 9, 6
+    T = 6
     x = torch.randn(B, T, I, device=dev, requires_grad=True)
     y = m(x)[0]
     y.sum().backward()
-    lengths = torch.tensor([6, 1, 3, 6, 2, 5, 4, 6, 1])
+    lengths = torch.tensor([6, 1, 3, 6, 2, 5, 4, 6, 1] * 9)[:B]
     xp = pack_padded_sequence(x.detach().requires_grad_(True), lengths, batch_first=True, enforce_sorted=False)
     yp = m(xp)[0]
     yp.data.sum().backward()
     with torch.no_grad():
         m.eval()(x)
     torch.cuda.synchronize()
-    print(kind, H, "ok", flush=True)
+    print(kind, H, B, "ok", flush=True)
 if sys.argv[1:] == ["rnn"]:
     sys.exit(0)
 # round 2: the fused shells (LayerNorm prologue + pooled gradient under autograd, attention pooling fwd/bwd, Softmax+CE,
