@@ -2,8 +2,9 @@
 ``b200rnn.TrainStep`` (zero_grad -> forward -> Softmax+CrossEntropy -> backward incl. dx -> FlatAdamW, one CUDA graph)
 vs ``oracle.ref_models.RefAudio / RefText`` + ``nn.CrossEntropyLoss`` on the Softmax outputs + ``torch.optim.AdamW``
 with the reference's parameter grouping (audio_gru_whole.py:161-201, 247-255, 307-308; text_bilstm_whole.py:154-193,
-303-304), three consecutive steps at the BASELINE c2 / c3 sizes. Dropout forced to 0 in train mode (RNG streams cannot
-match bit for bit).
+303-304), three consecutive steps at the BASELINE c2 / c3 sizes. Dropout is forced to 0 in train mode here, because
+torch's dropout RNG cannot be reproduced. The same steps with the encoders' dropout at the reference's 0.5 are checked
+with the library's own masks in test_gpu_dropout_exact.py.
 
 Tolerances: loss <= 1e-5 abs per step; first-step gradients <= 1e-4 of the largest entry; parameters after three steps:
 Adam's update is ~lr * sign(g) for |g| >> eps, so elements whose gradient is below the fp32 noise floor may move the
