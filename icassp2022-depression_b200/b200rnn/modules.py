@@ -192,9 +192,11 @@ class _B200RNNBase(nn.Module):
         """
         need_grad = torch.is_grad_enabled() and (input.requires_grad or any(p.requires_grad for p in self.parameters())
                                                  or (ln is not None and any(p.requires_grad for p in ln.parameters())))
+        # the folded LayerNorm needs the tensor-core layer-0 projection, whose N = gates * hidden_size must be a
+        # multiple of 128 (not so for a GRU with hidden_size 64)
         shape_ok = (input.is_cuda and input.dim() == 3 and
                     (ln is None or (self.input_size in (128, 256, 512, 1024) and ln.elementwise_affine and
-                                    ln.bias is not None)))
+                                    ln.bias is not None and (self._gates * self.hidden_size) % 128 == 0)))
         if need_grad and shape_ok and not isinstance(input, nn.utils.rnn.PackedSequence):
             # training graph: LayerNorm forward+backward folded around the layer-0 GEMMs, pooled gradient broadcast
             # inside the BPTT kernel (no [T,B,H] output gradient, no LN(x) autograd tensor)

@@ -55,8 +55,8 @@ int check_desc(const b200rnn_desc* d, Dims* o) {
               d->num_dirs);
     return B200RNN_ERR_INVALID;
   }
-  if (d->hidden_size != 128 && d->hidden_size != 256) {
-    set_error("hidden_size %d unsupported: the sm_100a persistent kernels are built for 128 and 256",
+  if (d->hidden_size != 64 && d->hidden_size != 128 && d->hidden_size != 256 && d->hidden_size != 512) {
+    set_error("hidden_size %d unsupported: the sm_100a persistent kernels are built for 64, 128, 256 and 512",
               d->hidden_size);
     return B200RNN_ERR_UNSUPPORTED;
   }
@@ -586,8 +586,11 @@ B200RNN_API int b200rnn_backward_fused(const b200rnn_desc* desc, const float* x,
         float* hnS = S + sl.b_tc_hn;   // [TB][H]   (GRU: dn * r)
         const TcOperand opX{xS, xS + d.TB * (size_t)Il, (long long)Il, true};
         // the tcgen05 epilogue stores float4: a gradient target that is not 16-byte aligned (a view into a caller's
-        // flat bucket behind an odd-sized tensor) takes the FFMA GEMM below instead of failing
-        const bool tc_wih = dw_ih && aligned_to(dw_ih, 16), tc_whh = dw_hh && aligned_to(dw_hh, 16) && d.T > 1;
+        // flat bucket behind an odd-sized tensor) takes the FFMA GEMM below instead of failing. The dW_hh GEMMs are
+        // H wide (N = H) and the tensor-core tile is 128 wide: H = 64 takes the FFMA GEMM for them. The other two have
+        // N = Il (a multiple of 128 here) and contract over T*B or G*H, which the tiles' zero fill covers at any size.
+        const bool tc_wih = dw_ih && aligned_to(dw_ih, 16);
+        const bool tc_whh = dw_hh && aligned_to(dw_hh, 16) && d.T > 1 && d.H % 128 == 0;
         float* Cx = nullptr;
         RowMap cx_rows = simple_rows(1);
         bool tc_dx = false;

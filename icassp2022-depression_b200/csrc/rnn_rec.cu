@@ -59,7 +59,7 @@ struct RecCfg {
   static constexpr int CPS = ROT ? HS / CW : 1;     // chunks per source slice (ROT)
   static constexpr int SPC = ROT ? 1 : CW / HS;     // source slices per chunk (!ROT)
   static constexpr int NBAR = 1 + 2 * C;            // [0] weights, [1 + buf*C + src] state slices
-  static constexpr size_t BAR_BYTES = 256;
+  static constexpr size_t BAR_BYTES = (NBAR * 8 <= 256) ? 256 : 512;  // 512 only for the 16-CTA clusters (H = 512)
   static constexpr size_t W_BYTES = (size_t)NSM * HS * H * sizeof(float);
   static constexpr size_t FWD_SMEM = W_BYTES + (size_t)2 * BS * H * sizeof(float) + BAR_BYTES;
   static constexpr size_t BWD_SMEM = W_BYTES + (size_t)2 * BS * GH * sizeof(float) + BAR_BYTES;
@@ -390,6 +390,10 @@ __global__ void __launch_bounds__(RecCfg<MODE, H, C, BS, KL, UPL, RG>::NT, 1)
   using Cfg = RecCfg<MODE, H, C, BS, KL, UPL, RG>;
   using LM = LaneMap<KL, UPL, BS>;
   static_assert(RG <= 1, "the backward kernel keeps at most one gate block in registers");
+  // Streamed variant: the last gate block is too large for the register file (H / BS floats per thread, over 64) and
+  // is read from global memory (L2: W_hh is small and read by every cluster) in every step instead. Only the LSTM
+  // H = 512 backward uses it: there the 16 CTAs of a cluster would each need 256 KB of transposed W_hh on chip.
+  constexpr bool STREAM = RG == 1 && UPL * (H / KL) > 64;
   constexpr int G = Cfg::G, GH = Cfg::GH, HS = Cfg::HS, NT = Cfg::NT, UPW = Cfg::UPW, NSM = Cfg::NSM;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float* W_s = reinterpret_cast<float*>(smem_raw);   // [NSM][HS][H] transposed gate blocks
@@ -424,7 +428,8 @@ __global__ void __launch_bounds__(RecCfg<MODE, H, C, BS, KL, UPL, RG>::NT, 1)
   for (int i = tid; i < 2 * BS * GH; i += NT) d_s[i] = 0.f;
   const int rot = Cfg::ROT ? (int)rank * CPS : 0;
   float wreg[1][UPL][H / KL];
-  load_resident<RG, KL, UPL, BS, H>(w_prep + (size_t)NSM * HS * H, HS, (long long)w * UPW, rot, lane, wreg);
+  if constexpr (!STREAM)
+    load_resident<RG, KL, UPL, BS, H>(w_prep + (size_t)NSM * HS * H, HS, (long long)w * UPW, rot, lane, wreg);
   ptx::mbar_wait(&bars[0], 0);
   __syncthreads();
   ptx::cluster_sync_all();
@@ -576,6 +581,9 @@ __global__ void __launch_bounds__(RecCfg<MODE, H, C, BS, KL, UPL, RG>::NT, 1)
         if (g < NSM)
           dots_chunk2<1, 0, KL, UPL, BS, H, GH>(W_s + (size_t)g * HS * H, 0, w * UPW, wreg, d_buf + g * H, c, ca,
                                                 lane, acc2);
+        else if constexpr (STREAM)
+          dots_chunk2<1, 0, KL, UPL, BS, H, GH>(w_prep + (size_t)NSM * HS * H, 0, w * UPW, wreg, d_buf + g * H, c,
+                                                ca, lane, acc2);
         else
           dots_chunk2<1, 1, KL, UPL, BS, H, GH>(W_s, 0, 0, wreg, d_buf + g * H, c, ca, lane, acc2);
       }
@@ -606,7 +614,7 @@ __global__ void __launch_bounds__(RecCfg<MODE, H, C, BS, KL, UPL, RG>::NT, 1)
 // launchers
 // =================================================================================================
 template <typename K>
-int prepare_kernel(K kernel, size_t smem) {
+int prepare_kernel(K kernel, size_t smem, int C) {
   struct Done {
     const void* k;
     int dev;
@@ -619,6 +627,8 @@ int prepare_kernel(K kernel, size_t smem) {
   for (int i = 0; i < ndone; ++i)
     if (done[i].k == (const void*)kernel && done[i].dev == dev) return B200RNN_OK;
   B200_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  // clusters above the portable size of 8 (the 16-CTA clusters of H = 512) have to be allowed explicitly
+  if (C > 8) B200_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
   if (ndone < 256) done[ndone++] = Done{(const void*)kernel, dev};
   return B200RNN_OK;
 }
@@ -626,7 +636,7 @@ int prepare_kernel(K kernel, size_t smem) {
 template <typename K, typename P>
 int launch_clustered(K kernel, const P& params, int nslices, int nclusters, int C, int NT, size_t smem,
                      cudaStream_t stream, int prof_kind) {
-  int rc = prepare_kernel(kernel, smem);
+  int rc = prepare_kernel(kernel, smem, C);
   if (rc) return rc;
   ProfScope prof(prof_kind, stream);
   cudaLaunchConfig_t cfg = {};
@@ -662,7 +672,7 @@ int max_active_clusters(K kernel, int C, int NT, size_t smem) {
     for (int i = 0; i < ncache; ++i)
       if (cache[i].k == (const void*)kernel && cache[i].dev == dev) return cache[i].n;
   }
-  if (prepare_kernel(kernel, smem) != B200RNN_OK) return 0;
+  if (prepare_kernel(kernel, smem, C) != B200RNN_OK) return 0;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)(C * 148), 1, 1);
   cfg.blockDim = dim3((unsigned)NT, 1, 1);
@@ -684,6 +694,16 @@ int max_active_clusters(K kernel, int C, int NT, size_t smem) {
   return n;
 }
 
+// A non-portable cluster (C > 8) needs C free SMs in one GPC: a device partitioned below that (MIG, a green context)
+// reports room for no cluster at all. Such a launch would fail; report it as unsupported instead.
+template <typename K>
+bool cluster_fits(K kernel, int C, int NT, size_t smem, int* rc) {
+  if (max_active_clusters(kernel, C, NT, smem) > 0) return true;
+  set_error("recurrence: this device cannot hold one %d-CTA cluster (%zu B shared memory per CTA)", C, smem);
+  *rc = B200RNN_ERR_UNSUPPORTED;
+  return false;
+}
+
 template <int MODE, int H, int C, int BS, int KL, int UPL, int RG, bool PB = false>
 bool try_fwd(const RecFwdParams& p, cudaStream_t s, bool force, int* rc) {
   using Cfg = RecCfg<MODE, H, C, BS, KL, UPL, RG>;
@@ -697,6 +717,7 @@ bool try_fwd(const RecFwdParams& p, cudaStream_t s, bool force, int* rc) {
     fprintf(stderr, "[b200rnn] fwd cfg C=%d BS=%d KL=%d UPL=%d RG=%d: need %d clusters, capacity %d, smem %zu\n", C, BS,
             KL, UPL, RG, nclusters, max_active_clusters(k, C, Cfg::NT, Cfg::FWD_SMEM), (size_t)Cfg::FWD_SMEM);
   if (!force && nclusters > max_active_clusters(k, C, Cfg::NT, Cfg::FWD_SMEM)) return false;
+  if (C > 8 && !cluster_fits(k, C, Cfg::NT, Cfg::FWD_SMEM, rc)) return true;
   *rc = launch_clustered(k, p, nslices, nclusters, C, Cfg::NT, Cfg::FWD_SMEM, s, PROF_REC_FWD);
   return true;
 }
@@ -709,6 +730,7 @@ bool try_bwd(RecBwdParams& p, cudaStream_t s, bool force, int* rc) {
   const int nslices = (p.B + BS - 1) / BS;
   const int nclusters = nslices * p.D;
   if (!force && nclusters > max_active_clusters(k, C, Cfg::NT, Cfg::BWD_SMEM)) return false;
+  if (C > 8 && !cluster_fits(k, C, Cfg::NT, Cfg::BWD_SMEM, rc)) return true;
   // transposed, per-CTA contiguous copy of W_hh for this cluster width
   for (int d = 0; d < p.D; ++d) {
     whh_prep_kernel<<<148, dim3(32, 8), 0, s>>>(p.w_hh[d], p.w_prep[d], Cfg::G, H, C);
@@ -770,7 +792,29 @@ int launch_rec_fwd(const RecFwdParams& p, cudaStream_t s) {
     try_fwd<B200RNN_LSTM, 128, 4, 8, 16, 2, 1>(p, s, true, &rc);
     return rc;
   }
-  set_error("recurrence: unsupported (mode=%d, hidden_size=%d); built for hidden_size 128 and 256", p.mode,
+  // H = 64: the H = 128 configs at half the width (H % (4*KL) == 0 caps KL at 16); W_hh is 48 / 64 KB per direction
+  if (p.mode == B200RNN_GRU && p.H == 64) {
+    if (try_fwd<B200RNN_GRU, 64, 2, 4, 16, 4, 1>(p, s, false, &rc)) return rc;
+    try_fwd<B200RNN_GRU, 64, 2, 8, 16, 2, 1>(p, s, true, &rc);
+    return rc;
+  }
+  if (p.mode == B200RNN_LSTM && p.H == 64) {
+    if (try_fwd<B200RNN_LSTM, 64, 2, 4, 16, 4, 1>(p, s, false, &rc)) return rc;
+    try_fwd<B200RNN_LSTM, 64, 2, 8, 16, 2, 1>(p, s, true, &rc);
+    return rc;
+  }
+  // H = 512: 16-CTA clusters (HS = 32 units per CTA), the largest that exists; nothing wider to fall back to, so the
+  // batch runs in as many waves as it needs. GRU: all three gate blocks in shared memory (213 504 B); LSTM: three in
+  // shared memory (229 888 B), the fourth in registers (64 floats per thread)
+  if (p.mode == B200RNN_GRU && p.H == 512) {
+    try_fwd<B200RNN_GRU, 512, 16, 4, 16, 4, 0>(p, s, true, &rc);
+    return rc;
+  }
+  if (p.mode == B200RNN_LSTM && p.H == 512) {
+    try_fwd<B200RNN_LSTM, 512, 16, 8, 16, 2, 1>(p, s, true, &rc);
+    return rc;
+  }
+  set_error("recurrence: unsupported (mode=%d, hidden_size=%d); built for hidden_size 64, 128, 256 and 512", p.mode,
             p.H);
   return B200RNN_ERR_UNSUPPORTED;
 }
@@ -801,7 +845,29 @@ int launch_rec_bwd(RecBwdParams& p, cudaStream_t s) {
     try_bwd<B200RNN_LSTM, 128, 4, 8, 32, 4, 1>(p, s, true, &rc);
     return rc;
   }
-  set_error("recurrence backward: unsupported (mode=%d, hidden_size=%d)", p.mode, p.H);
+  if (p.mode == B200RNN_GRU && p.H == 64) {
+    if (try_bwd<B200RNN_GRU, 64, 2, 4, 16, 4, 1>(p, s, false, &rc)) return rc;
+    try_bwd<B200RNN_GRU, 64, 2, 8, 16, 2, 1>(p, s, true, &rc);
+    return rc;
+  }
+  if (p.mode == B200RNN_LSTM && p.H == 64) {
+    if (try_bwd<B200RNN_LSTM, 64, 2, 4, 16, 4, 1>(p, s, false, &rc)) return rc;
+    try_bwd<B200RNN_LSTM, 64, 2, 8, 16, 2, 1>(p, s, true, &rc);
+    return rc;
+  }
+  // H = 512, 16-CTA clusters. GRU: two transposed gate blocks in shared memory, one in registers (229 888 B). LSTM: no
+  // config holds all four blocks on chip (256 KB per CTA); three sit in shared memory and the fourth is streamed from
+  // L2 in every step (rec_bwd_kernel's STREAM variant, 64 KB per CTA per step), 2 batch rows per cluster (229 888 B)
+  if (p.mode == B200RNN_GRU && p.H == 512) {
+    try_bwd<B200RNN_GRU, 512, 16, 8, 32, 4, 1>(p, s, true, &rc);
+    return rc;
+  }
+  if (p.mode == B200RNN_LSTM && p.H == 512) {
+    try_bwd<B200RNN_LSTM, 512, 16, 2, 8, 4, 1>(p, s, true, &rc);
+    return rc;
+  }
+  set_error("recurrence backward: unsupported (mode=%d, hidden_size=%d); built for hidden_size 64, 128, 256 and 512",
+            p.mode, p.H);
   return B200RNN_ERR_UNSUPPORTED;
 }
 

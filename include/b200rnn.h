@@ -65,7 +65,7 @@ typedef struct b200rnn_desc {
   int32_t batch;       /* B */
   int32_t seq_len;     /* T */
   int32_t input_size;  /* I  (layer-0 feature width)                                        */
-  int32_t hidden_size; /* H  (supported: 128, 256)                                          */
+  int32_t hidden_size; /* H  (supported: 64, 128, 256, 512)                                 */
   int32_t num_layers;  /* L                                                                 */
   int32_t num_dirs;    /* D  (1, or 2 = bidirectional)                                      */
   int32_t training;    /* 1: module is in train() mode => inter-layer dropout is applied      */
